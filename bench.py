@@ -856,6 +856,18 @@ def run_own(args, rank, local_rank, world):
             comp_d, own_d = out_dep[(step_no[0] - 1) & 1], lay_dep[(step_no[0] - 1) & 1]
             closer = int(((comp_d != own_d)).sum().item())
             log(f"[rank 0] composite: {closer} pixels taken from instance layers")
+        if args.dump_outputs and rank == 0:
+            # what the last timed step handed its caller, before the untimed frames below overwrite it: ICP points and normals,
+            # ray points and the shaded image of rank 0's volume; at N > 1 rank 0's composite instead of its own image
+            out = {"points": points.view(H_, W, 4), "normals": normals.view(H_, W, 4), "raycast_result": rs.raycastResult.view(H_, W, 4)}
+            if world == 1:
+                out["raycast_image"] = rs.raycastImage.view(H_, W, 4)
+            else:
+                out["composite_colour"], out["composite_depth"] = out_col[(step_no[0] - 1) & 1], out_dep[(step_no[0] - 1) & 1]
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, t in out.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), t.float().cpu().numpy())
+            log(f"[rank 0] wrote {', '.join(out)} of timed step {K - 1} to {args.dump_outputs}")
         # per-stage breakdown of a few extra frames (per-frame sync; not part of the timed region)
         eng.set_timing(1)
         stage = np.zeros(6)
@@ -1117,7 +1129,11 @@ def main():
     ap.add_argument("--hires-frames", type=int, default=24,
                     help="frames of the 4 mm roofline-stress stream (0 = skip; > 64 = the stream at length, e.g. 2000 for configs[4])")
     ap.add_argument("--decay-blocks", type=int, default=2000000, help="allocated blocks of the Decay() sweep, configs[3] (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32), to compare two builds on the same inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,18 +1,32 @@
 """The drop-in, exercised through the reference's own C++ objects and virtual interfaces
 (oracle/itm_harness.cpp): (1) the B200 shim classes behind ITMSceneReconstructionEngine /
 IITMVisualisationEngine produce exactly the oracle's state; (2) the UNMODIFIED reference CUDA engines,
-built for sm_100a, agree with it on the order-free invariants (the reference is nondeterministic and
-compiled with --use_fast_math, SURVEY finding 4, so bit-exactness is not defined against it)."""
+built for sm_100a, agree with the B200 engine on the order-free invariants (the reference is nondeterministic and
+compiled with --use_fast_math, SURVEY finding 4, so bit-exactness is not defined against it).
+
+(1) and the patched ITMMainEngine need the harness libraries built from the reference's sources (oracle/build_ref.sh,
+integration/build_patched.sh). For (2) the reference CUDA engines' outputs on these inputs are stored in
+tests/golden/itm_reference_cuda.npz and the B200 engine is compared against them; with DYNSLAM_RECORD_PINS=1 and the
+harness built, the reference engines are run through it, compared against the B200 shim and the stored outputs rewritten."""
 import ctypes as C
+import os
 
 import numpy as np
 import pytest
+import torch
 
-from dynslam_b200 import abi, synth
+from dynslam_b200 import abi, engine as E, synth
 from tests import harnesslib as HL
 from tests import hostlib as H
+from tests.refpins import RECORD
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not HL.available(), reason="oracle/_ref/libitmharness.so not built")]
+pytestmark = pytest.mark.gpu
+needs_harness = pytest.mark.skipif(not HL.available(), reason="oracle/_ref/libitmharness.so not built (needs the reference's sources)")
+REF_CUDA = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "itm_reference_cuda.npz")
+# what is stored of the reference's outputs (each file under tests/golden/ stays well below 1 MB): 64 voxels of each of 300 sampled
+# blocks, which pixels the raycast hit and 4096 sampled ray points; of the view builder's output the invalid mask, the borders and
+# 16384 sampled pixels
+PICK_BLOCKS, VOXELS_PER_BLOCK, RAY_SAMPLES, VIEW_SAMPLES = 300, 64, 4096, 16384
 
 NB, NE = 0x100000, 0x80000
 SCALE, NUM_BLOCKS, FRAMES = 0.25, 32768, 6
@@ -37,6 +51,7 @@ def _oracle_run(frames, decay):
     return vol
 
 
+@needs_harness
 def test_shim_through_itmlib_objects_is_bit_exact():
     frames = _frames()
     decay = (2, 2)
@@ -63,8 +78,70 @@ def _by_pos(state):
     return {tuple(int(c) for c in hs["pos"][i]): int(hs["ptr"][i]) for i in used}
 
 
-def test_reference_cuda_build_agrees_on_order_free_invariants():
-    frames = _frames()
+def _engine_run(frames):
+    """The frames through the B200 engine's ITMLib-shaped API in the harness's order (AllocateSceneFromDepth,
+    IntegrateIntoScene, CreateExpectedDepths, CreateICPMaps), no decay: hash table, voxels, ray points and counters."""
+    w, h = frames[0][0].shape[1], frames[0][0].shape[0]
+    scene = E.Scene(E.SceneParams(), NUM_BLOCKS, NB, NE, device="cuda:0")
+    eng = E.Engine(scene, (w, h))
+    reco, vis = E.SceneReconstructionEngine(eng), E.VisualisationEngine(eng, scene)
+    rs = vis.CreateRenderState((w, h))
+    reco.ResetScene(scene)
+    points = torch.zeros(h * w * 4, dtype=torch.float32, device="cuda:0")
+    normals = torch.zeros(h * w * 4, dtype=torch.float32, device="cuda:0")
+    for depth, rgb, M, proj in frames:
+        gv = E.View(torch.from_numpy(depth).cuda(), torch.from_numpy(rgb).cuda(), M, proj)
+        reco.AllocateSceneFromDepth(scene, gv, rs)
+        reco.IntegrateIntoScene(scene, gv, rs)
+        vis.CreateExpectedDepths(E.make_camera(M, proj), rs)
+        vis.CreateICPMaps(gv, rs, points, normals)
+    g, r = scene.to_host(), rs.to_host()
+    rays = rs.raycastResult.cpu().numpy().reshape(h, w, 4)
+    return dict(hash=g["hash"], voxels=g["voxels"], rays=rays), dict(noVisibleBlocks=int(r["noVisibleBlocks"]))
+
+
+def _sample(n, k, seed):
+    """the fixed, seeded sample of k of n indices that tests/golden/itm_reference_cuda.npz stores values at"""
+    return np.sort(np.random.RandomState(seed).choice(n, size=min(k, n), replace=False))
+
+
+def _agrees_with_reference_cuda(ref, own, own_counters):
+    """ref: the reference CUDA engines' allocated block positions and visible-block count, sampled voxels of sampled blocks,
+    which pixels their raycast hit and the ray points at sampled pixels (the layout of tests/golden/itm_reference_cuda.npz)."""
+    pr = {tuple(int(c) for c in p) for p in ref["positions"]}
+    po = _by_pos(own)
+    common = pr & set(po)
+    # same set of allocated block positions, up to same-frame bucket races / skipped contended steps in the reference
+    assert len(common) >= 0.995 * max(len(pr), len(po)), (len(pr), len(po), len(common))
+    nv_r, nv_o = int(ref["noVisibleBlocks"]), own_counters["noVisibleBlocks"]
+    assert abs(nv_r - nv_o) <= 0.01 * nv_o + 2
+    # per-position voxel contents: weights identical, TSDF within 1e-5 (float) where the nearest-pixel lookup agrees;
+    # fast-math projection flips a few lookups, so allow a small fraction of outliers and report it
+    vox = _sample(512, VOXELS_PER_BLOCK, 1)
+    pick = [k for k, p in enumerate(ref["pick"]) if tuple(int(c) for c in p) in po]
+    assert len(pick) >= 0.99 * len(ref["pick"])
+    n = bad_w = bad_sdf = 0
+    for k in pick:
+        p = tuple(int(c) for c in ref["pick"][k])
+        a_w, a_sdf = ref["pick_w_depth"][k * vox.size:(k + 1) * vox.size], ref["pick_sdf"][k * vox.size:(k + 1) * vox.size]
+        b = own["voxels"][po[p] * 512:(po[p] + 1) * 512][vox]
+        n += vox.size
+        bad_w += int((a_w != b["w_depth"]).sum())
+        d = np.abs(a_sdf.astype(np.float32) / 32767.0 - b["sdf"].astype(np.float32) / 32767.0)
+        bad_sdf += int((d > 1e-5 + 1.0 / 32767.0).sum())     # 1 LSB of the short quantisation + 1e-5
+    assert bad_w / n < 0.03 and bad_sdf / n < 0.03, (bad_w / n, bad_sdf / n)   # measured on B200: ~1.3 % / ~1.1 %
+    # the raycast images agree on almost every pixel
+    rays_o = own["rays"].reshape(-1, 4)
+    found_r, found_o = np.unpackbits(ref["ray_found"])[:rays_o.shape[0]].astype(bool), rays_o[:, 3] > 0
+    assert (found_r == found_o).mean() > 0.98
+    px = _sample(rays_o.shape[0], RAY_SAMPLES, 2)
+    both = found_r[px] & found_o[px]
+    assert np.abs(ref["ray_xyz"][both] - rays_o[px][both][:, :3]).max(axis=1).mean() < 0.05   # voxel units
+
+
+def _record_reference_cuda(frames):
+    """Runs the reference CUDA engines and the B200 shim through the harness, checks them against each other and returns the
+    reference's outputs in the stored layout."""
     w, h = frames[0][0].shape[1], frames[0][0].shape[0]
     res = {}
     for impl in (HL.REFERENCE_CUDA, HL.B200_SHIM):
@@ -73,36 +150,39 @@ def test_reference_cuda_build_agrees_on_order_free_invariants():
             hs.process_frame(depth, rgb, M, decay=None)
         res[impl] = (hs.download(), hs.counters())
         hs.close()
-    (ref, rc), (own, oc) = res[HL.REFERENCE_CUDA], res[HL.B200_SHIM]
-    pr, po = _by_pos(ref), _by_pos(own)
-    common = set(pr) & set(po)
-    # same set of allocated block positions, up to same-frame bucket races / skipped contended steps in the reference
-    assert len(common) >= 0.995 * max(len(pr), len(po)), (len(pr), len(po), len(common))
-    assert abs(rc["noVisibleBlocks"] - oc["noVisibleBlocks"]) <= 0.01 * oc["noVisibleBlocks"] + 2
-    # per-position voxel contents: weights identical, TSDF within 1e-5 (float) where the nearest-pixel lookup agrees;
-    # fast-math projection flips a few lookups, so allow a small fraction of outliers and report it
+    (ref, rc), (shim, sc) = res[HL.REFERENCE_CUDA], res[HL.B200_SHIM]
+    pr, ps = _by_pos(ref), _by_pos(shim)
     rng = np.random.RandomState(0)
-    pick = [sorted(common)[i] for i in rng.choice(len(common), size=min(1500, len(common)), replace=False)]
-    n = bad_w = bad_sdf = 0
-    for p in pick:
-        a = ref["voxels"][pr[p] * 512:(pr[p] + 1) * 512]
-        b = own["voxels"][po[p] * 512:(po[p] + 1) * 512]
-        n += 512
-        bad_w += int((a["w_depth"] != b["w_depth"]).sum())
-        d = np.abs(a["sdf"].astype(np.float32) / 32767.0 - b["sdf"].astype(np.float32) / 32767.0)
-        bad_sdf += int((d > 1e-5 + 1.0 / 32767.0).sum())     # 1 LSB of the short quantisation + 1e-5
-    assert bad_w / n < 0.03 and bad_sdf / n < 0.03, (bad_w / n, bad_sdf / n)   # measured on B200: ~1.3 % / ~1.1 %
-    # the raycast images agree on almost every pixel
-    found_r, found_o = ref["rays"][..., 3] > 0, own["rays"][..., 3] > 0
-    assert (found_r == found_o).mean() > 0.98
-    both = found_r & found_o
-    assert np.abs(ref["rays"][both][:, :3] - own["rays"][both][:, :3]).max(axis=1).mean() < 0.05   # voxel units
+    common = sorted(set(pr) & set(ps))
+    pick = [common[i] for i in rng.choice(len(common), size=min(PICK_BLOCKS, len(common)), replace=False)]
+    vox = _sample(512, VOXELS_PER_BLOCK, 1)
+    blocks = np.concatenate([ref["voxels"][pr[p] * 512:(pr[p] + 1) * 512][vox] for p in pick])
+    rays = ref["rays"].reshape(-1, 4)
+    stored = dict(positions=np.array(sorted(pr), dtype=np.int16), noVisibleBlocks=np.int64(rc["noVisibleBlocks"]),
+                  pick=np.array(pick, dtype=np.int16), pick_sdf=blocks["sdf"].copy(), pick_w_depth=blocks["w_depth"].copy(),
+                  ray_found=np.packbits(rays[:, 3] > 0), ray_xyz=rays[_sample(rays.shape[0], RAY_SAMPLES, 2), :3].copy())
+    _agrees_with_reference_cuda(stored, shim, sc)
+    return stored
+
+
+def test_reference_cuda_build_agrees_on_order_free_invariants():
+    frames = _frames()
+    own, oc = _engine_run(frames)
+    if RECORD and HL.available():
+        ref = _record_reference_cuda(frames)
+        stored = dict(np.load(REF_CUDA)) if os.path.exists(REF_CUDA) else {}
+        stored.update({"engines/" + k: v for k, v in ref.items()})
+        np.savez_compressed(REF_CUDA, **stored)
+    with np.load(REF_CUDA) as z:
+        ref = {k.split("/", 1)[1]: z[k] for k in z.files if k.startswith("engines/")}
+    _agrees_with_reference_cuda(ref, own, oc)
 
 
 def test_view_builder_through_itmlib_objects():
     """ITMViewBuilder_B200 behind the abstract ITMViewBuilder, called the way ITMMainEngine::ProcessFrame calls it
-    (host ITMUChar4Image / ITMShortImage in): close to the oracle (libm vs CUDA exp), zero border exactly; the
-    reference's ITMViewBuilder_CUDA (fast-math exp and division) agrees within 1e-4 relative."""
+    (host ITMUChar4Image / ITMShortImage in), and the B200 engine's own UpdateView: close to the oracle (libm vs CUDA exp),
+    zero border exactly; the reference's ITMViewBuilder_CUDA (fast-math exp and division; its output stored in
+    tests/golden/itm_reference_cuda.npz) agrees within 1e-4 relative."""
     from tests import viewlib
     raw, rgb = viewlib.raw_kitti_frame(scale=0.5)
     h, w = raw.shape
@@ -114,22 +194,47 @@ def test_view_builder_through_itmlib_objects():
     want, scratch = np.zeros((h, w), np.float32), np.zeros((h, w), np.float32)
     L.oracle_update_view(H.vptr(raw), w, h, C.byref(calib), H.vptr(want), H.vptr(scratch), None, None)
     got = {}
-    for impl in (HL.B200_SHIM, HL.REFERENCE_CUDA):
-        vb = HL.ViewBuilderHarness(impl, w, h, proj)
-        first = vb.update_view(raw, rgb)
-        again = vb.update_view(raw, rgb)                    # second frame through the same builder: same result
-        assert np.array_equal(first, again)
-        got[impl] = first
-        vb.close()
-    for impl, tol in ((HL.B200_SHIM, 5e-6), (HL.REFERENCE_CUDA, 1e-4)):
+    eng = E.Engine(E.Scene(E.SceneParams(), 2048, 0x800, 0x400, "cuda:0"), (w, h))
+    vb = E.ViewBuilder(eng, E.make_view_calib(intrinsics_d=proj))
+    d_raw = torch.from_numpy(np.ascontiguousarray(raw, dtype=np.int16)).cuda()
+    first, again = (torch.full((h, w), 3.0, dtype=torch.float32, device="cuda") for _ in range(2))
+    vb.UpdateView(first, d_raw)
+    vb.UpdateView(again, d_raw)                             # second frame through the same builder: same result
+    assert torch.equal(first, again)
+    got["engine"] = first.cpu().numpy()
+    if RECORD and HL.available():
+        for impl in (HL.B200_SHIM, HL.REFERENCE_CUDA):
+            vbh = HL.ViewBuilderHarness(impl, w, h, proj)
+            first = vbh.update_view(raw, rgb)
+            again = vbh.update_view(raw, rgb)
+            assert np.array_equal(first, again)
+            got[impl] = first
+            vbh.close()
+        r = got[HL.REFERENCE_CUDA]
+        stored = dict(np.load(REF_CUDA)) if os.path.exists(REF_CUDA) else {}
+        stored.update({"view_builder/invalid": np.packbits((r == -1.0).reshape(-1)),
+                       "view_builder/depth_sample": r.reshape(-1)[_sample(r.size, VIEW_SAMPLES, 3)].copy(),
+                       "view_builder/border": np.concatenate([r[:2].ravel(), r[-2:].ravel(), r[:, :2].ravel(), r[:, -2:].ravel()])})
+        np.savez_compressed(REF_CUDA, **stored)
+    with np.load(REF_CUDA) as z:
+        ref = {k.split("/", 1)[1]: z[k] for k in z.files if k.startswith("view_builder/")}
+    for impl in ("engine", HL.B200_SHIM):
+        if impl not in got:
+            continue
         g = got[impl]
         assert ((g == -1.0) == (want == -1.0)).all()
         err = np.abs(g.astype(np.float64) - want) / np.maximum(1.0, np.abs(want))
-        assert err.max() <= tol, (impl, err.max())
+        assert err.max() <= 5e-6, (impl, err.max())
         assert (g[:2] == 0).all() and (g[-2:] == 0).all() and (g[:, :2] == 0).all() and (g[:, -2:] == 0).all()
+    # the reference's output: same invalid mask, within 1e-4 at the sampled pixels, zero border
+    assert (np.unpackbits(ref["invalid"])[:want.size].astype(bool) == (want == -1.0).reshape(-1)).all()
+    px = _sample(want.size, VIEW_SAMPLES, 3)
+    err = np.abs(ref["depth_sample"].astype(np.float64) - want.reshape(-1)[px]) / np.maximum(1.0, np.abs(want.reshape(-1)[px]))
+    assert err.max() <= 1e-4, err.max()
+    assert (ref["border"] == 0).all()
 
 
-@pytest.mark.skipif(not HL.patched_available(), reason="oracle/_ref/libitmpatched.so not built (integration/build_patched.sh)")
+@pytest.mark.skipif(not HL.patched_available(), reason="oracle/_ref/libitmpatched.so not built (integration/build_patched.sh; needs the reference's sources)")
 def test_patched_main_engine_runs_both_backends():
     """The binding a maintainer adds, compiled and RUN: integration/itmlib_b200.patch applied to the reference's ITMLib, the
     whole library rebuilt, and the reference's own top-level object — ITMMainEngine, the base class of DynSLAM's

@@ -1,6 +1,7 @@
 """CPU: dynslam_b200/csrc/hostio.c — the on-disk formats either side of the path (SURVEY 8(f) rank 4) — against
 (1) the reference's own ReadFilePFM (src/pfmLib), ReadMask (PrecomputedSegmentationProvider.cpp) and ITMMesh::WriteOBJ, compiled
-    from the reference tree into oracle/_ref/libioref.so (oracle/build_ref.sh, oracle/ref_io_driver.cpp): byte for byte; and
+    from the reference tree into oracle/_ref/libioref.so (oracle/build_ref.sh, oracle/ref_io_driver.cpp): byte for byte, against
+    their outputs stored in tests/golden/reference_pins.json (tests/refpins.py); and
 (2) known answers for the OpenCV XML depth dump and the max-depth clamp (OpenCV itself is not available to produce a pin)."""
 import ctypes as C
 import os
@@ -10,9 +11,9 @@ import pytest
 
 from dynslam_b200 import abi, formats
 from tests import hostlib as H
+from tests.refpins import pin
 
 IOREF_SO = os.path.join(H.ROOT, "oracle", "_ref", "libioref.so")
-needs_ref = pytest.mark.skipif(not os.path.exists(IOREF_SO), reason="oracle/_ref/libioref.so not built (needs /root/reference at build time)")
 
 
 def ioref():
@@ -33,7 +34,6 @@ def write_pfm(path, a, little=True, crlf=False):
         f.write(np.ascontiguousarray(a[::-1]).astype("<f4" if little else ">f4").tobytes())
 
 
-@needs_ref
 @pytest.mark.parametrize("shape,little,crlf", [((37, 53), True, False), ((16, 9), False, False), ((12, 20, 3), True, True), ((5, 7, 3), False, False)])
 def test_pfm_equals_reference_reader(tmp_path, shape, little, crlf):
     rng = np.random.default_rng(3)
@@ -42,11 +42,13 @@ def test_pfm_equals_reference_reader(tmp_path, shape, little, crlf):
     write_pfm(p, a, little, crlf)
     got = formats.read_pfm(p)
     assert got.shape == a.shape and np.array_equal(got, a)                 # row 0 at the top, byte order undone
-    L = ioref()
-    w, h, b = C.c_int(), C.c_int(), C.c_int()
-    ref = np.zeros(a.size, np.float32)
-    assert L.ref_read_pfm(p.encode(), C.byref(w), C.byref(h), C.byref(b), ref.ctypes.data, ref.size) == 0
-    assert (h.value, w.value) == a.shape[:2] and ref.tobytes() == got.tobytes()
+
+    def ref_read():
+        w, h, b = C.c_int(), C.c_int(), C.c_int()
+        ref = np.zeros(a.size, np.float32)
+        rc = ioref().ref_read_pfm(p.encode(), C.byref(w), C.byref(h), C.byref(b), ref.ctypes.data, ref.size)
+        return [rc, [h.value, w.value], ref]
+    pin(f"hostio/read_pfm/{'x'.join(map(str, shape))}-{'le' if little else 'be'}{'-crlf' if crlf else ''}", [0, list(a.shape[:2]), got], ref_read)
 
 
 def test_pfm_errors(tmp_path):
@@ -58,7 +60,6 @@ def test_pfm_errors(tmp_path):
         formats.read_pfm(str(p))
 
 
-@needs_ref
 def test_mask_txt_equals_reference_reader(tmp_path):
     rng = np.random.default_rng(5)
     m = (rng.uniform(size=(23, 31)) < 0.4).astype(np.float64)
@@ -66,24 +67,25 @@ def test_mask_txt_equals_reference_reader(tmp_path):
     np.savetxt(p, m)                                                        # numpy's default "%.18e" text dump, as the segmentation tool writes it
     got = formats.read_mask_txt(p, 31, 23)
     assert np.array_equal(got, m.astype(np.uint8))
-    L = ioref()
-    ref = np.zeros((23, 31), np.uint8)
-    assert L.ref_read_mask(p.encode(), 31, 23, ref.ctypes.data) == 0
-    assert np.array_equal(ref, got)
+
+    def ref_read(w, h):
+        ref = np.zeros((23, 31), np.uint8)
+        return [ioref().ref_read_mask(p.encode(), w, h, ref.ctypes.data), ref]
+    pin("hostio/read_mask/float_dump", [0, got], lambda: ref_read(31, 23))
     # integer dumps and values other than 0 / 1 are truncated to a byte the same way
     np.savetxt(p, (m * 2.7), fmt="%.3f")
     got = formats.read_mask_txt(p, 31, 23)
-    assert L.ref_read_mask(p.encode(), 31, 23, ref.ctypes.data) == 0 and np.array_equal(ref, got) and got.max() == 2
+    assert got.max() == 2
+    pin("hostio/read_mask/fixed_dump", [0, got], lambda: ref_read(31, 23))
     # wrong size: both refuse
     with pytest.raises(RuntimeError):
         formats.read_mask_txt(p, 30, 23)
-    assert L.ref_read_mask(p.encode(), 30, 23, ref.ctypes.data) == -3
+    pin("hostio/read_mask/too_narrow", -3, lambda: ref_read(30, 23)[0])
     with pytest.raises(RuntimeError):
         formats.read_mask_txt(p, 31, 22)
-    assert L.ref_read_mask(p.encode(), 31, 22, ref.ctypes.data) == -3
+    pin("hostio/read_mask/too_short", -3, lambda: ref_read(31, 22)[0])
 
 
-@needs_ref
 def test_obj_equals_reference_writer(tmp_path):
     rng = np.random.default_rng(9)
     n = 257
@@ -94,12 +96,15 @@ def test_obj_equals_reference_writer(tmp_path):
         t[k] = rng.uniform(0, 1, (n, 3)).astype(np.float32)
     ours, ref = str(tmp_path / "ours.obj"), str(tmp_path / "ref.obj")
     formats.write_obj(ours, t, n, 512)
-    assert ioref().ref_write_obj(ref.encode(), t.ctypes.data, n, 16) == 0        # 16 blocks -> noMaxTriangles 512
-    assert open(ours, "rb").read() == open(ref, "rb").read()
+
+    def ref_write():
+        rc = ioref().ref_write_obj(ref.encode(), t.ctypes.data, n, 16)        # 16 blocks -> noMaxTriangles 512
+        return [rc, open(ref, "rb").read()]
+    pin("hostio/write_obj", [0, open(ours, "rb").read()], ref_write)
     # more triangles than the mesh can hold: the reference throws, we raise with its text
     with pytest.raises(RuntimeError, match="Too many triangles"):
         formats.write_obj(ours, t, n, 100)
-    assert ioref().ref_write_obj(ref.encode(), t.ctypes.data, 600, 16) == -3
+    pin("hostio/write_obj/too_many_triangles", -3, lambda: ioref().ref_write_obj(ref.encode(), t.ctypes.data, 600, 16))
 
 
 def test_depth_xml_and_clamp_known_answers(tmp_path):
